@@ -70,7 +70,26 @@ def parse():
                     help="like --timeline but for 3 steps of the end-to-end loop (Trainer.train_step_pipelined, pinned H2D + D2H)")
     ap.add_argument("--worker-streams", type=int, default=None,
                     help="concurrent CUDA streams for logical workers sharing a GPU (default: the JobConfig default)")
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy: params.npy (the PS's "
+                         "fp32 parameter arena, a fixed seeded sample when larger than 48 MB) and metrics.npy (loss, Prec@1, "
+                         "Prec@5, fp64)")
     return ap.parse_args()
+
+
+DUMP_MAX_PARAMS = 12 * 2 ** 20          # fp32 elements (48 MB): params.npy + metrics.npy stay under 64 MB
+
+
+def _dump_outputs(out_dir, params, metrics):
+    """Write the outputs of the last timed step.  Inputs and initial parameters are seeded, so two builds run with the same
+    arguments can be compared file for file; an arena above DUMP_MAX_PARAMS is sampled at the same positions every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    p = params.detach().float().cpu().numpy()
+    if p.size > DUMP_MAX_PARAMS:
+        p = p[np.sort(np.random.default_rng(0).choice(p.size, DUMP_MAX_PARAMS, replace=False))]
+    np.save(os.path.join(out_dir, "params.npy"), p)
+    np.save(os.path.join(out_dir, "metrics.npy"), np.asarray(metrics, dtype=np.float64))
 
 
 def _write_timeline(path, trainer, rank, barrier, pipelined=False):
@@ -168,14 +187,51 @@ def main() -> int:
     if sampler:
         sampler.start()
 
-    def mean_loss(m):
+    def mean_loss(m, key="loss"):
         vals = [None] * world
         if world > 1:
-            dist.all_gather_object(vals, m.get("loss") if m else None)
+            dist.all_gather_object(vals, m.get(key) if m else None)
         else:
-            vals = [m.get("loss") if m else None]
+            vals = [m.get(key) if m else None]
         vals = [v for v in vals if v is not None]
         return sum(vals) / len(vals) if vals else None
+
+    # ------------------------------------------------------------------ value: device-timed, no host sync in the loop
+    # Runs first, from the seeded initial model: what --dump-outputs writes is the state after exactly warmup + steps training
+    # steps, whether or not the e2e loop runs.  (The headline's 3 liars out-vote r=3 groups and the model diverges; its
+    # parameters overflow fp32 after about 40 steps.)  The engines capture their CUDA graph on the third step, so at least
+    # three warm-up steps keep the capture out of the timed window.
+    cfg.data_on_device = True
+    for _ in range(max(a.warmup, 3)):
+        trainer.train_step_async()
+    barrier()
+    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    s.record()
+    for _ in range(a.steps):
+        trainer.train_step_async()
+    e.record()
+    barrier()
+    ms = reduce_max(s.elapsed_time(e))
+    launches = reduce_sum(float(getattr(eng, "kernels_per_step", 0) * a.steps))
+    # device-side timeline (spin-wait stamps): how long workers wait for parameters / the PS waits for gradients per step
+    trace = eng.wait_trace(min(a.steps, 16)) if hasattr(eng, "wait_trace") else {}
+    traces = [None] * world
+    if world > 1:
+        dist.all_gather_object(traces, trace)
+    else:
+        traces = [trace]
+    ww = [t["worker_wait_ms"] for t in traces if t and "worker_wait_ms" in t]
+    breakdown = {"ps_wait_for_grads_ms": next((t["ps_wait_ms"] for t in traces if t and "ps_wait_ms" in t), None),
+                 "worker_wait_for_params_ms_mean": sum(ww) / len(ww) if ww else None,
+                 "worker_wait_for_params_ms_min": min(ww) if ww else None} if traces and any(traces) else None
+    m = eng.read_metrics()
+    if a.dump_outputs:
+        # mean over the ranks hosting workers; the PS's arena (rank 0) is the master copy every worker trains on
+        metrics = [mean_loss(m, k) for k in ("loss", "prec1", "prec5")]
+        if rank == 0:
+            _dump_outputs(a.dump_outputs, eng.master_params(), [float("nan") if v is None else v for v in metrics])
+    if a.timeline:
+        _write_timeline(a.timeline, trainer, rank, barrier)
 
     # ------------------------------------------------------------------ e2e: public API, pinned H2D + D2H every step
     e2e = None
@@ -209,35 +265,7 @@ def main() -> int:
                "api": "Trainer.train_step_pipelined() + drain()",
                "result_read": "every step's loss/Prec@k is copied device->host into pinned memory and read by the host one "
                               "step later (while the next step runs); the last one is drained inside the timed region"}
-
-    # ------------------------------------------------------------------ value: device-timed, no host sync in the loop
-    cfg.data_on_device = True
-    for _ in range(a.warmup):
-        trainer.train_step_async()
-    barrier()
-    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    s.record()
-    for _ in range(a.steps):
-        trainer.train_step_async()
-    e.record()
-    barrier()
     clocks = sampler.stop() if sampler else None
-    ms = reduce_max(s.elapsed_time(e))
-    launches = reduce_sum(float(getattr(eng, "kernels_per_step", 0) * a.steps))
-    # device-side timeline (spin-wait stamps): how long workers wait for parameters / the PS waits for gradients per step
-    trace = eng.wait_trace(min(a.steps, 16)) if hasattr(eng, "wait_trace") else {}
-    traces = [None] * world
-    if world > 1:
-        dist.all_gather_object(traces, trace)
-    else:
-        traces = [trace]
-    ww = [t["worker_wait_ms"] for t in traces if t and "worker_wait_ms" in t]
-    breakdown = {"ps_wait_for_grads_ms": next((t["ps_wait_ms"] for t in traces if t and "ps_wait_ms" in t), None),
-                 "worker_wait_for_params_ms_mean": sum(ww) / len(ww) if ww else None,
-                 "worker_wait_for_params_ms_min": min(ww) if ww else None} if traces and any(traces) else None
-    m = eng.read_metrics()
-    if a.timeline:
-        _write_timeline(a.timeline, trainer, rank, barrier)
     trainer.close()
 
     # ------------------------------------------------------------------ sanity point: the code tolerates what it promises
