@@ -9,16 +9,21 @@
 // place, and stores the fresh parameters directly into every worker's parameter arena -- with one NVLS
 // `multimem.st` through a multicast mapping when available, otherwise with unicast peer stores -- and the
 // last CTA raises the step-stamped `params_ready` flag on every worker.  No NCCL call.
+//
+// MODE 3 adds the coordinate-wise robust rules (Yin et al., ICML 2018): trimmed mean and median.  Each output
+// element depends only on the P values at the same position, so the rule runs inside this streaming kernel and
+// is bucket-pipelined like the mean.
 #include "common.cuh"
 
 struct UpdateArgs {
   // gradient source ---------------------------------------------------------------------------
-  int mode;                       // 0: select-sum over `select` table; 1: cyclic recombination; 2: real per-tensor weights
+  int mode;                       // 0: select-sum over `select` table; 1: cyclic recombination; 2: real per-tensor weights;
+                                  // 3: coordinate-wise trimmed sum over the K slots (median / trimmed mean)
   const float* grad_in;           // mode 0: [P][slot_stride] fp32 ; mode 1: [n][2*slot_stride] complex64
   long long slot_stride;          // elements (fp32 words for mode 0, complex elements for mode 1)
   const int* select;              // mode 0: [K][T] worker slot to read for (k, tensor); null -> rows 0..K-1 for all tensors
   int K;                          // mode 0: rows summed per tensor ; mode 1: n workers
-  float scale;                    // 1/K (mean, vote), 1 (krum, median vector), 1/n (cyclic)
+  float scale;                    // 1/K (mean, vote), 1 (krum, median vector), 1/n (cyclic), 1/(K - 2 trim) (mode 3)
   const float2* recomb;           // mode 1: [T][n] recombination vector v (float2 = complex64); mode 2: float [T][K] weights
   TileView tv;
   // optimizer ---------------------------------------------------------------------------------
@@ -37,9 +42,79 @@ struct UpdateArgs {
   unsigned int* done_counter;
   FlagList flags;                 // params_ready flags (peer pointers); value written = step + 1
   int tile_begin, tile_end;       // bucket of tiles to update + broadcast (tile_end == 0: whole arena)
+  int trim;                       // mode 3: values dropped at each end of every coordinate's sorted column (2 trim < K)
 };
 
-template <int MODE>
+// Order-preserving map float -> uint32: unsigned comparison of keys = numeric order of the floats, -0 just below +0.
+// Every NaN (either sign, any payload) becomes one canonical key above +Inf, the order of np.sort.  Padding slots of the
+// sorting network get 0xffffffff, above every real value including NaN.
+#define DRC_KEY_NAN 0xfffffffeu
+#define DRC_KEY_PAD 0xffffffffu
+__device__ __forceinline__ unsigned int order_key(float x) {
+  const unsigned int u = __float_as_uint(x);
+  if (x != x) return DRC_KEY_NAN;
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float key_value(unsigned int k) {
+  return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+
+// Batcher's odd-even merge sort on N (a power of two) keys, ascending: 19 compare-exchanges for N = 8, 63 for N = 16.
+// The comparator list is built at compile time, so the network unrolls into straight-line min / max pairs on registers.
+template <int N>
+struct SortNet {
+  static constexpr int kMax = N * N;              // more than enough room for the comparators of N <= 16
+  int n = 0, lo[kMax] = {}, hi[kMax] = {};
+  constexpr SortNet() {
+    for (int p = 1; p < N; p <<= 1)
+      for (int k = p; k >= 1; k >>= 1)
+        for (int j = k % p; j + k < N; j += 2 * k)
+          for (int i = 0; i < k && i + j + k < N; ++i)
+            if ((i + j) / (2 * p) == (i + j + k) / (2 * p)) { lo[n] = i + j; hi[n] = i + j + k; ++n; }
+  }
+};
+
+template <int N>
+__device__ __forceinline__ void sort_network(unsigned int (&v)[N]) {
+  constexpr SortNet<N> net;
+#pragma unroll
+  for (int c = 0; c < net.n; ++c) {
+    const unsigned int x = v[net.lo[c]], y = v[net.hi[c]];
+    v[net.lo[c]] = min(x, y);
+    v[net.hi[c]] = max(x, y);
+  }
+}
+
+// MODE 3: sort each of the thread's 4 coordinates over the P = K slots and sum the kept values s_{trim} .. s_{P-trim-1}
+// (0-based) in ascending order.  MAXP is the network size (8 or 16), chosen from P by the launcher.
+template <int MAXP>
+__device__ __forceinline__ float4 trimmed_sum(const float* __restrict__ src, long long stride, int K, int trim) {
+  unsigned int key[4][MAXP];
+#pragma unroll
+  for (int k = 0; k < MAXP; ++k) {
+    if (k < K) {
+      const float4 v = ld_f4(reinterpret_cast<const float4*>(src + k * stride));
+      key[0][k] = order_key(v.x); key[1][k] = order_key(v.y); key[2][k] = order_key(v.z); key[3][k] = order_key(v.w);
+    } else {
+      key[0][k] = key[1][k] = key[2][k] = key[3][k] = DRC_KEY_PAD;
+    }
+  }
+  // bit k set: s_k is summed (one uniform mask instead of two compares per slot keeps both instantiations free of spills)
+  const unsigned int kept = ((1u << (K - trim)) - 1u) & ~((1u << trim) - 1u);
+  float s[4];
+#pragma unroll
+  for (int e = 0; e < 4; ++e) {
+    sort_network<MAXP>(key[e]);
+    float acc = 0.f;
+#pragma unroll
+    for (int k = 0; k < MAXP; ++k)
+      if ((kept >> k) & 1u) acc += key_value(key[e][k]);
+    s[e] = acc;
+  }
+  return make_float4(s[0], s[1], s[2], s[3]);
+}
+
+template <int MODE, int MAXP = 0>
 __global__ void __launch_bounds__(DRC_THREADS) aggregate_update_kernel(const __grid_constant__ UpdateArgs a) {
   const HyperParams hp = *a.hp;
   const unsigned long long step = *a.step_ptr;
@@ -62,6 +137,8 @@ __global__ void __launch_bounds__(DRC_THREADS) aggregate_update_kernel(const __g
         float4 v = ld_f4(reinterpret_cast<const float4*>(a.grad_in + slot * a.slot_stride + idx));
         g.x += v.x; g.y += v.y; g.z += v.z; g.w += v.w;
       }
+    } else if constexpr (MODE == 3) {
+      g = trimmed_sum<MAXP>(a.grad_in + idx, a.slot_stride, a.K, a.trim);
     } else if (MODE == 2) {
       const float* wts = reinterpret_cast<const float*>(a.recomb);    // geometric median: sum_k w[tensor][k] * g_k
       for (int k = 0; k < a.K; ++k) {
@@ -134,6 +211,12 @@ extern "C" int drc_aggregate_update(const UpdateArgs* args, int grid, cudaStream
   if (args->ndst > DRC_MAX_DST || args->flags.n > DRC_MAX_DST) return (int)cudaErrorInvalidValue;
   if (args->mode == 0) aggregate_update_kernel<0><<<grid, DRC_THREADS, 0, stream>>>(*args);
   else if (args->mode == 2) aggregate_update_kernel<2><<<grid, DRC_THREADS, 0, stream>>>(*args);
+  else if (args->mode == 3) {
+    if (args->K < 1 || args->trim < 0 || 2 * args->trim >= args->K) return (int)cudaErrorInvalidValue;
+    if (args->K <= 8) aggregate_update_kernel<3, 8><<<grid, DRC_THREADS, 0, stream>>>(*args);
+    else if (args->K <= 16) aggregate_update_kernel<3, 16><<<grid, DRC_THREADS, 0, stream>>>(*args);
+    else return (int)cudaErrorInvalidValue;
+  }
   else aggregate_update_kernel<1><<<grid, DRC_THREADS, 0, stream>>>(*args);
   return (int)cudaGetLastError();
 }

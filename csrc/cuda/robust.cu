@@ -19,6 +19,10 @@
 // Krum -- reference: double Python loop of np.linalg.norm per tensor (baseline_master.py:278-296).  Here one
 // pass produces all P(P-1)/2 squared distances per tensor, a one-thread-per-tensor kernel scores and selects,
 // and the winner row goes through the fused select + SGD + broadcast kernel.
+//
+// Multi-Krum (Blanchard et al., NeurIPS 2017) shares the distances and the scores: the selection keeps the m rows
+// with the lowest scores (ties to the lower slot), and the fused kernel averages them with its select-sum (MODE 0),
+// which reads only the selected rows.  m = 1 is Krum.
 #include "common.cuh"
 
 #define GM_MAXP DRC_MAX_WORKERS
@@ -193,7 +197,8 @@ __global__ void __launch_bounds__(DRC_THREADS) pair_dist_kernel(const __grid_con
 struct KrumSelectArgs {
   double* pair_d2;                // consumed and zeroed
   int T, P, s;
-  int* select;                    // [T] winning worker slot
+  int* select;                    // [m][T] selected worker slots, ascending per tensor (m = 1: the Krum winner)
+  int m;                          // rows kept (1 <= m <= P)
 };
 
 __global__ void krum_select_kernel(const __grid_constant__ KrumSelectArgs a) {
@@ -203,7 +208,7 @@ __global__ void krum_select_kernel(const __grid_constant__ KrumSelectArgs a) {
   double* d2 = a.pair_d2 + (long long)t * npairs;
   int keep = a.P - a.s - 2;
   if (keep < 0) keep = 0;
-  double best = 0.0; int best_i = 0;
+  double scores[KRUM_MAXP];
   for (int i = 0; i < a.P; ++i) {
     double nb[KRUM_MAXP]; int c = 0;
     for (int j = 0; j < a.P; ++j) {
@@ -214,9 +219,21 @@ __global__ void krum_select_kernel(const __grid_constant__ KrumSelectArgs a) {
     for (int x = 1; x < c; ++x) { double k = nb[x]; int y = x - 1; while (y >= 0 && nb[y] > k) { nb[y + 1] = nb[y]; --y; } nb[y + 1] = k; }
     double score = 0.0;
     for (int x = 0; x < keep && x < c; ++x) score += nb[x];
-    if (i == 0 || score < best) { best = score; best_i = i; }
+    scores[i] = score;
   }
-  a.select[t] = best_i;
+  // m rounds of Krum's argmin (first row, then strictly lower scores) over the rows not taken yet: the first round is
+  // exactly the Krum selection, non-finite scores included
+  unsigned int taken = 0u;
+  for (int r = 0; r < a.m; ++r) {
+    double best = 0.0; int best_i = -1;
+    for (int i = 0; i < a.P; ++i) {
+      if ((taken >> i) & 1u) continue;
+      if (best_i < 0 || scores[i] < best) { best = scores[i]; best_i = i; }
+    }
+    taken |= 1u << best_i;
+  }
+  for (int i = 0, c = 0; i < a.P; ++i)
+    if ((taken >> i) & 1u) a.select[(long long)(c++) * a.T + t] = i;
   for (int q = 0; q < npairs; ++q) d2[q] = 0.0;
 }
 
@@ -226,7 +243,7 @@ extern "C" int drc_pair_dist(const PairDistArgs* args, int grid, cudaStream_t st
   return (int)cudaGetLastError();
 }
 extern "C" int drc_krum_select(const KrumSelectArgs* args, cudaStream_t stream) {
-  if (args->P > KRUM_MAXP) return (int)cudaErrorInvalidValue;
+  if (args->P > KRUM_MAXP || args->m < 1 || args->m > args->P) return (int)cudaErrorInvalidValue;
   krum_select_kernel<<<(args->T + 63) / 64, 64, 0, stream>>>(*args);
   return (int)cudaGetLastError();
 }

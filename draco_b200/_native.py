@@ -75,7 +75,7 @@ class UpdateArgs(C.Structure):
                 ("scale", C.c_float), ("recomb", ptr), ("tv", TileView), ("params", ptr), ("momentum", ptr),
                 ("exp_avg_sq", ptr), ("max_exp_avg_sq", ptr), ("hp", ptr), ("step_ptr", ptr), ("first_step", u64), ("grad_out", ptr), ("mc_params", ptr),
                 ("dst", ptr * MAX_DST), ("ndst", C.c_int), ("done_counter", ptr), ("flags", FlagList),
-                ("tile_begin", C.c_int), ("tile_end", C.c_int)]
+                ("tile_begin", C.c_int), ("tile_end", C.c_int), ("trim", C.c_int)]
 
 
 class StreamPushArgs(C.Structure):
@@ -125,7 +125,7 @@ class PairDistArgs(C.Structure):
 
 
 class KrumSelectArgs(C.Structure):
-    _fields_ = [("pair_d2", ptr), ("T", C.c_int), ("P", C.c_int), ("s", C.c_int), ("select", ptr)]
+    _fields_ = [("pair_d2", ptr), ("T", C.c_int), ("P", C.c_int), ("s", C.c_int), ("select", ptr), ("m", C.c_int)]
 
 
 def _maybe_build() -> None:

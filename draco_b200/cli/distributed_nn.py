@@ -21,8 +21,21 @@ import sys
 from ..config import add_fit_args, config_from_args
 
 
+RULES = """aggregation rules (per parameter tensor, P workers, f = --worker-fail):
+  --approach maj_vote --mode maj_vote       repetition-code majority vote (Draco)
+  --approach cyclic                         cyclic-code decode (Draco)
+  --approach baseline --mode normal         mean
+  --approach baseline --mode geometric_median
+  --approach baseline --mode krum           Krum
+  --approach baseline --mode multi_krum     mean of the P - f best Krum rows       (P >= 2f + 3)
+  --approach baseline --mode coord_median   coordinate-wise median                 (P >= 2f + 1)
+  --approach baseline --mode trimmed_mean   coordinate-wise mean without the f lowest and f highest values  (P >= 2f + 1)
+"""
+
+
 def main(argv=None) -> int:
-    ap = add_fit_args(argparse.ArgumentParser(description="Draco on B200 (draco_b200)"))
+    ap = add_fit_args(argparse.ArgumentParser(description="Draco on B200 (draco_b200)", epilog=RULES,
+                                              formatter_class=argparse.RawDescriptionHelpFormatter))
     ap.add_argument("--launch", type=int, default=0, help="spawn this many local processes with torchrun semantics")
     ap.add_argument("--master-port", type=int, default=29511)
     args = ap.parse_args(argv)

@@ -104,6 +104,33 @@ def krum(slots: np.ndarray, s: int) -> np.ndarray:
     return np.asarray(slots, dtype=np.float64)[krum_index(slots, s)]
 
 
+def multi_krum_indices(slots: np.ndarray, s: int, m: int) -> List[int]:
+    """Multi-Krum (Blanchard et al., NeurIPS 2017): the m rows with the lowest Krum scores (ties to the lower slot), in
+    ascending slot order.  The aggregate is their mean; m = 1 is Krum.  Defined for finite inputs."""
+    X = np.asarray(slots, dtype=np.float64)
+    P = X.shape[0]
+    keep = max(P - s - 2, 0)
+    d2 = ((X[:, None, :] - X[None, :, :]) ** 2).sum(axis=2)
+    scores = np.array([np.sort(np.delete(d2[i], i))[:keep].sum() for i in range(P)])
+    return sorted(int(i) for i in np.argsort(scores, kind="stable")[:m])
+
+
+def trimmed_mean(slots: np.ndarray, b: int) -> np.ndarray:
+    """Coordinate-wise trimmed mean (Yin et al., ICML 2018): sort every coordinate's P values with ``np.sort`` (NaN of either
+    sign after +Inf), drop the b lowest and the b highest, average the rest.  Up to b non-finite values per coordinate are
+    trimmed away."""
+    X = np.sort(np.asarray(slots, dtype=np.float64), axis=0)
+    P = X.shape[0]
+    assert 0 <= 2 * b < P
+    return X[b: P - b].sum(axis=0) / (P - 2 * b)
+
+
+def coordinate_median(slots: np.ndarray) -> np.ndarray:
+    """Coordinate-wise median: the trimmed mean that keeps the middle value (odd P) or averages the middle two (even P) --
+    ``np.median`` on finite inputs."""
+    return trimmed_mean(slots, (np.asarray(slots).shape[0] - 1) // 2)
+
+
 def sgd_momentum_step(p: np.ndarray, buf: np.ndarray, g: np.ndarray, lr: float, momentum: float,
                       weight_decay: float = 0.0, dampening: float = 0.0, nesterov: bool = False,
                       first_step: bool = False) -> Tuple[np.ndarray, np.ndarray]:

@@ -11,7 +11,8 @@ from dataclasses import asdict, dataclass
 from typing import Optional
 
 APPROACHES = ("baseline", "maj_vote", "cyclic")
-MODES = ("normal", "geometric_median", "krum", "maj_vote")
+MODES = ("normal", "geometric_median", "krum", "maj_vote", "coord_median", "trimmed_mean", "multi_krum")
+ROBUST_NVL_MAXP = 16            # P limit of coord_median / trimmed_mean / multi_krum on nvl (register budget of their kernels)
 ERR_MODES = ("rev_grad", "constant", "random", "omniscient", "none")
 TRANSPORTS = ("nvl", "nccl", "nccl_flat", "gloo")
 
@@ -101,6 +102,18 @@ class JobConfig:
                                  f"divides num_workers more evenly")
         if self.no_cuda:
             self.transport = "gloo"
+        if self.approach == "baseline" and self.mode in ("coord_median", "trimmed_mean", "multi_krum"):
+            P, f = self.num_workers, self.worker_fail
+            if f < 0:
+                raise ValueError(f"--mode {self.mode} needs --worker-fail >= 0")
+            if self.mode in ("coord_median", "trimmed_mean") and P < 2 * f + 1:
+                raise ValueError(f"--mode {self.mode} needs num_workers >= 2*worker_fail + 1 (got {P} workers, "
+                                 f"worker_fail {f}): a majority of every coordinate's values must be honest")
+            if self.mode == "multi_krum" and P < 2 * f + 3:
+                raise ValueError(f"--mode multi_krum needs num_workers >= 2*worker_fail + 3 (got {P} workers, worker_fail {f})")
+            if self.transport == "nvl" and P > ROBUST_NVL_MAXP:
+                raise ValueError(f"--mode {self.mode} on --transport nvl handles at most {ROBUST_NVL_MAXP} workers (got {P}); "
+                                 f"use --transport nccl for more")
         if self.compress and self.transport == "nvl" and self.err_mode == "omniscient":
             raise ValueError("--err-mode omniscient reads the honest slots in PS memory while they arrive; with --compress-grad "
                              "compress they only exist after the PS unpacked them -- pass --compress-grad None")
@@ -153,7 +166,8 @@ def add_fit_args(parser: argparse.ArgumentParser) -> argparse.ArgumentParser:
     a("--profile-phases", action="store_true", default=d.profile_phases,
       help="time the reference's phases (Comm / Comp / Encode / Method / Update) with CUDA events each step; eager mode")
     a("--network", type=str, default=d.network)
-    a("--mode", type=str, default=d.mode, help="normal | geometric_median | krum (baseline); normal | maj_vote (maj_vote)")
+    a("--mode", type=str, default=d.mode,
+      help="normal | geometric_median | krum | coord_median | trimmed_mean | multi_krum (baseline); normal | maj_vote (maj_vote)")
     a("--dataset", type=str, default=d.dataset)
     a("--comm-type", type=str, default=d.comm_type)
     a("--err-mode", type=str, default=d.err_mode, help="rev_grad | constant | random | omniscient | none")

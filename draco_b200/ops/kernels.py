@@ -134,15 +134,20 @@ def aggregate_update(layout: ArenaLayout, grad_in: Addr, slot_stride: int, *, pa
                      recomb: Addr = None, first_step: int = 1, grad_out: Addr = None, mc_params: Addr = None,
                      dst: Sequence[Addr] = (), flags: Sequence[Addr] = (), grid: Optional[int] = None,
                      tile_range: Optional[tuple] = None, weights: Addr = None, exp_avg_sq: Addr = None,
-                     max_exp_avg_sq: Addr = None) -> None:
-    """Fused aggregate (select-sum, cyclic recombination, or real per-tensor ``weights`` [T, K]) + optimizer step (SGD-momentum, or
-    Adam / AMSGrad when the hyper-parameter block says so: ``momentum`` = first moment, ``exp_avg_sq`` / ``max_exp_avg_sq`` = second
-    moment / its running maximum) + parameter broadcast + flags."""
+                     max_exp_avg_sq: Addr = None, trim: Optional[int] = None) -> None:
+    """Fused aggregate (select-sum, cyclic recombination, real per-tensor ``weights`` [T, K], or with ``trim`` the coordinate-wise
+    trimmed sum: per element, the K slot values sorted ascending (NaN last) without the ``trim`` lowest and highest, summed) +
+    optimizer step (SGD-momentum, or Adam / AMSGrad when the hyper-parameter block says so: ``momentum`` = first moment,
+    ``exp_avg_sq`` / ``max_exp_avg_sq`` = second moment / its running maximum) + parameter broadcast + flags.  Everything is
+    multiplied by ``scale`` before the optimizer step: 1 / (K - 2 trim) makes the trimmed sum a trimmed mean / median."""
     a = N.UpdateArgs()
-    a.mode = 1 if recomb is not None else (2 if weights is not None else 0)
+    a.mode = 1 if recomb is not None else (2 if weights is not None else (3 if trim is not None else 0))
     if weights is not None:
-        assert recomb is None and select is None
+        assert recomb is None and select is None and trim is None
         recomb = weights
+    if trim is not None:
+        assert recomb is None and select is None
+        a.trim = trim
     a.grad_in = addr(grad_in)
     a.slot_stride = slot_stride
     a.select = addr(select)
@@ -296,12 +301,14 @@ def geometric_median_weights(layout: ArenaLayout, grad_in: Addr, slot_stride: in
 
 
 def krum_select(layout: ArenaLayout, grad_in: Addr, slot_stride: int, P: int, s: int, pair_d2: torch.Tensor,
-                select: torch.Tensor) -> None:
-    """``pair_d2``: zeroed fp64 [T, P*(P-1)/2] scratch (left zeroed); ``select``: int32 [T] out (winning slot)."""
+                select: torch.Tensor, m: int = 1) -> None:
+    """Krum (m = 1) or multi-Krum selection.  ``pair_d2``: zeroed fp64 [T, P*(P-1)/2] scratch (left zeroed); ``select``: int32
+    [m, T] out, the m lowest-scoring slots of every tensor in ascending slot order ([T] is accepted for m = 1)."""
+    assert 1 <= m <= P and select.numel() == m * layout.ntensors and select.dtype == torch.int32
     lib = N.cuda()
     pa = N.PairDistArgs(addr(grad_in), slot_stride, P, layout.tile_view(select.device), pair_d2.data_ptr())
     N.check(lib.drc_pair_dist(C.byref(pa), stream_grid(layout, 4), _stream()), "pair_dist")
-    ka = N.KrumSelectArgs(pair_d2.data_ptr(), layout.ntensors, P, s, select.data_ptr())
+    ka = N.KrumSelectArgs(pair_d2.data_ptr(), layout.ntensors, P, s, select.data_ptr(), m)
     N.check(lib.drc_krum_select(C.byref(ka), _stream()), "krum_select")
 
 

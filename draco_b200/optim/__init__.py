@@ -17,7 +17,7 @@ from typing import Iterable, List, Sequence
 import numpy as np
 import torch
 
-_MODES = ("normal", "geometric_median", "maj_vote", "cyclic", "krum")
+_MODES = ("normal", "geometric_median", "maj_vote", "cyclic", "krum", "coord_median", "trimmed_mean", "multi_krum")
 
 
 def _as_tensor(g, like: torch.Tensor) -> torch.Tensor:

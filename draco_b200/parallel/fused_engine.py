@@ -39,7 +39,7 @@ from ..ops import kernels as K
 from ..utils.metrics import PhaseTimer, limit_host_threads, wait_event
 from .arena import ArenaLayout
 from .placement import Placement
-from .ps import FusedPS, build_codes, select_rule
+from .ps import COORDINATE_RULES, FusedPS, build_codes, select_rule
 from .symm import SymmContext
 from .worker import WorkerCompute, make_model
 
@@ -79,7 +79,7 @@ class FusedEngine:
         self.compress = bool(cfg.compress)
         self.overlap_push = cfg.overlap_push and not self.cyclic and not self.compress
         # PS pipelining: decode + apply + broadcast each gradient bucket as soon as all workers pushed it
-        self.pipeline_ps = (self.overlap_push and cfg.pipeline_ps and select_rule(cfg) in ("mean", "vote")
+        self.pipeline_ps = (self.overlap_push and cfg.pipeline_ps and select_rule(cfg) in ("mean", "vote") + COORDINATE_RULES
                             and cfg.err_mode != "omniscient")
         self.push_stream = torch.cuda.Stream(device=device) if self.overlap_push else None
         ns = min(max(int(cfg.worker_streams), 1), len(self.local_workers))

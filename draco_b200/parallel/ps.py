@@ -26,12 +26,23 @@ from .arena import ArenaLayout
 def select_rule(cfg: JobConfig) -> str:
     """Aggregation rule of a job.  Mirrors the reference's dispatch: cyclic approach -> Fourier decode
     (cyclic_master.py:24); maj_vote approach -> vote only when ``--mode maj_vote``, plain mean for ``--mode normal``
-    (rep_master.py:118-129); baseline approach -> mean / geometric median / Krum by ``--mode`` (baseline_master.py:118-129)."""
+    (rep_master.py:118-129); baseline approach -> mean / geometric median / Krum by ``--mode`` (baseline_master.py:118-129), plus
+    the coordinate-wise median and trimmed mean (Yin et al., ICML 2018) and multi-Krum (Blanchard et al., NeurIPS 2017)."""
     if cfg.approach == "cyclic":
         return "cyclic"
     if cfg.approach == "maj_vote":
         return "vote" if cfg.mode == "maj_vote" else "mean"
-    return {"normal": "mean", "geometric_median": "geomedian", "krum": "krum"}.get(cfg.mode, "mean")
+    return {"normal": "mean", "geometric_median": "geomedian", "krum": "krum", "coord_median": "coord_median",
+            "trimmed_mean": "trimmed_mean", "multi_krum": "multi_krum"}.get(cfg.mode, "mean")
+
+
+COORDINATE_RULES = ("coord_median", "trimmed_mean")
+
+
+def coordinate_trim(rule: str, P: int, f: int) -> int:
+    """Values dropped at each end of every coordinate's sorted column: f for the trimmed mean, all but the middle one
+    (odd P) or two (even P) for the median."""
+    return (P - 1) // 2 if rule == "coord_median" else f
 
 
 def hyperparams_tensor(cfg: JobConfig, device) -> torch.Tensor:
@@ -69,9 +80,12 @@ class FusedPS:
             self.neq_mask = torch.zeros(G, T, dtype=torch.int32, device=device)
             self.winner_slot = torch.zeros(G, T, dtype=torch.int32, device=device)
             self.winner_member = torch.zeros(G, T, dtype=torch.int32, device=device)
-        elif self.rule == "krum":
+        elif self.rule in ("krum", "multi_krum"):
+            self.krum_m = self.P - cfg.worker_fail if self.rule == "multi_krum" else 1
             self.pair_d2 = torch.zeros(T, self.P * (self.P - 1) // 2, dtype=torch.float64, device=device)
-            self.select = torch.zeros(T, dtype=torch.int32, device=device)
+            self.select = torch.zeros(self.krum_m, T, dtype=torch.int32, device=device)
+        elif self.rule in COORDINATE_RULES:
+            self.trim = coordinate_trim(self.rule, self.P, cfg.worker_fail)
         elif self.rule == "geomedian":
             if self.P <= K.GEOMED_FAST_MAXP:      # weight-space Weiszfeld: 2 passes over the slab in total
                 self.gm = None
@@ -108,7 +122,7 @@ class FusedPS:
                       hp=self.hp, step_ptr=step_ptr,
                       done_counter=self.counters[0:1], first_step=1, grad_out=grad_out, mc_params=mc_params, dst=dst)
         n = 0
-        if buckets is not None and self.rule in ("mean", "vote"):
+        if buckets is not None and self.rule in ("mean", "vote") + COORDINATE_RULES:
             for bi, (t0, t1, idxs) in enumerate(buckets):
                 n += wait_bucket(bi)
                 fl = flags if bi == len(buckets) - 1 else []
@@ -120,6 +134,11 @@ class FusedPS:
                         n += before_update()
                     K.aggregate_update(L, self.grad_in, self.slot_stride, K=G, scale=1.0 / G, select=self.winner_slot,
                                        tile_range=(t0, t1), flags=fl, **common); n += 1
+                elif self.rule in COORDINATE_RULES:
+                    if bi == len(buckets) - 1:
+                        n += before_update()
+                    K.aggregate_update(L, self.grad_in, self.slot_stride, K=self.P, scale=1.0 / (self.P - 2 * self.trim),
+                                       trim=self.trim, tile_range=(t0, t1), flags=fl, **common); n += 1
                 else:
                     if bi == len(buckets) - 1:
                         n += before_update()
@@ -139,9 +158,13 @@ class FusedPS:
             K.vote(L, self.grad_in, self.slot_stride, self.group_table, self.neq_mask, self.winner_slot, self.winner_member); n += 2
             G = self.group_table.shape[0]
             _update(L, self.grad_in, self.slot_stride, K=G, scale=1.0 / G, select=self.winner_slot, **common); n += 1
-        elif self.rule == "krum":
-            K.krum_select(L, self.grad_in, self.slot_stride, self.P, self.cfg.worker_fail, self.pair_d2, self.select); n += 2
-            _update(L, self.grad_in, self.slot_stride, K=1, scale=1.0, select=self.select, **common); n += 1
+        elif self.rule in ("krum", "multi_krum"):
+            m = self.krum_m
+            K.krum_select(L, self.grad_in, self.slot_stride, self.P, self.cfg.worker_fail, self.pair_d2, self.select, m=m); n += 2
+            _update(L, self.grad_in, self.slot_stride, K=m, scale=1.0 / m, select=self.select, **common); n += 1
+        elif self.rule in COORDINATE_RULES:
+            _update(L, self.grad_in, self.slot_stride, K=self.P, scale=1.0 / (self.P - 2 * self.trim), trim=self.trim,
+                    **common); n += 1
         elif self.rule == "geomedian" and self.gm is None:
             K.geometric_median_weights(L, self.grad_in, self.slot_stride, self.P, self.pair_d2, self.gm_weights); n += 2
             _update(L, self.grad_in, self.slot_stride, K=self.P, scale=1.0, weights=self.gm_weights, **common); n += 1
@@ -263,13 +286,29 @@ class TorchPS:
                 break
         return m
 
-    def _krum_tensor(self, X: torch.Tensor) -> int:
+    def _krum_scores(self, X: torch.Tensor) -> torch.Tensor:
         d2 = torch.cdist(X.double(), X.double()).pow(2)
         P = X.shape[0]
         keep = max(P - self.cfg.worker_fail - 2, 0)
         d2 = d2 + torch.diag(torch.full((P,), float("inf"), dtype=d2.dtype, device=d2.device))
-        scores = d2.sort(dim=1).values[:, :keep].sum(1)
-        return int(scores.argmin())
+        return d2.sort(dim=1).values[:, :keep].sum(1)
+
+    def _krum_tensor(self, X: torch.Tensor) -> int:
+        return int(self._krum_scores(X).argmin())
+
+    def _multi_krum_tensor(self, X: torch.Tensor) -> torch.Tensor:
+        """Mean of the P - f lowest-scoring rows (ties to the lower slot), summed in ascending slot order."""
+        m = self.P - self.cfg.worker_fail
+        rows = sorted(torch.argsort(self._krum_scores(X), stable=True)[:m].tolist())
+        acc = X[rows[0]].clone()
+        for r in rows[1:]:
+            acc += X[r]
+        return acc / m
+
+    def _coordinate_tensor(self, X: torch.Tensor) -> torch.Tensor:
+        """Coordinate-wise trimmed mean / median: sort every column (NaN last), drop ``trim`` values at each end."""
+        b = coordinate_trim(self.rule, self.P, self.cfg.worker_fail)
+        return torch.sort(X, dim=0).values[b: self.P - b].sum(0) / (self.P - 2 * b)
 
     def _cyclic_tensor(self, R: torch.Tensor, f: torch.Tensor) -> torch.Tensor:
         """R: [n, d] complex64 -> Re(v^T R) / n with v from the C++ locator (N1 replacement)."""
@@ -300,6 +339,10 @@ class TorchPS:
                 g = acc / float(self.groups.num_groups)
             elif self.rule == "krum":
                 g = X[self._krum_tensor(X)]
+            elif self.rule == "multi_krum":
+                g = self._multi_krum_tensor(X)
+            elif self.rule in COORDINATE_RULES:
+                g = self._coordinate_tensor(X)
             elif self.rule == "geomedian":
                 g = self._geomedian_tensor(X)
             elif self.rule == "cyclic":
@@ -313,7 +356,8 @@ class TorchPS:
         self.apply(self.aggregate(slots))
 
     def apply(self, grads: List[torch.Tensor]) -> None:
-        mode = {"mean": "normal", "vote": "maj_vote", "krum": "krum", "geomedian": "geometric_median", "cyclic": "cyclic"}[self.rule]
+        mode = {"mean": "normal", "vote": "maj_vote", "krum": "krum", "geomedian": "geometric_median", "cyclic": "cyclic",
+                "coord_median": "coord_median", "trimmed_mean": "trimmed_mean", "multi_krum": "multi_krum"}[self.rule]
         self.optimizer.step(grads=grads, mode=mode)
 
 
