@@ -60,6 +60,12 @@ class OmniArgs(C.Structure):
                 ("magnitude", C.c_float), ("total", i64), ("done_counter", ptr), ("flag", ptr), ("step_ptr", ptr)]
 
 
+class CollusionArgs(C.Structure):
+    _fields_ = [("grad_in", ptr), ("slot_stride", i64), ("P", C.c_int), ("tv", TileView), ("tile_begin", C.c_int),
+                ("tile_end", C.c_int), ("adv_bitmap", ptr), ("adv_len", C.c_int), ("step_ptr", ptr), ("mode", C.c_int),
+                ("param", C.c_float)]
+
+
 class VoteArgs(C.Structure):
     _fields_ = [("grad_in", ptr), ("slot_stride", i64), ("group_table", ptr), ("G", C.c_int), ("max_r", C.c_int),
                 ("tv", TileView), ("neq_mask", ptr), ("tile_begin", C.c_int), ("tile_end", C.c_int)]
@@ -185,6 +191,7 @@ def cuda() -> C.CDLL:
         for name, args in {
             "drc_push_encode": [C.POINTER(PushArgs), C.c_int, st],
             "drc_omniscient": [C.POINTER(OmniArgs), C.c_int, st],
+            "drc_collude": [C.POINTER(CollusionArgs), C.c_int, st],
             "drc_vote_compare": [C.POINTER(VoteArgs), C.c_int, st],
             "drc_vote_resolve": [C.POINTER(ResolveArgs), st],
             "drc_aggregate_update": [C.POINTER(UpdateArgs), C.c_int, st],

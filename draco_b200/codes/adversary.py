@@ -13,13 +13,22 @@ Attack parity (src/model_ops/utils.py:3-23), ``mag = -100``:
   omniscient (north-star extension): g -> -k * mean(honest gradients); needs a view of the honest
              gradients so it is applied by the engine, not by the per-worker hook.
 
-The device implementation of the same hook lives in csrc/cuda/push_encode.cu; the integer codes
-below are shared with it.
+Colluding attacks, designed to defeat the robust baselines (see ``collude``).  Every liar of the step
+sends the same vector, built from the per-coordinate mean ``mu`` and unbiased standard deviation
+``sigma`` of the honest slots:
+  alie : g -> mu - z * sigma   "A Little Is Enough" (Baruch et al., NeurIPS 2019); z = ``alie_z_max``
+  ipm  : g -> -epsilon * mu    inner-product manipulation (Xie et al., UAI 2019)
+Both read every honest gradient, so they are applied where all of them meet: at the parameter server,
+after the gradients arrived and before the aggregation rule runs (csrc/cuda/collude.cu).
+
+The device implementation of the per-worker hook lives in csrc/cuda/push_encode.cu; the integer codes
+below are shared with it and with collude.cu.
 """
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import List, Optional
+from statistics import NormalDist
+from typing import List, Optional, Sequence
 
 import numpy as np
 
@@ -31,6 +40,9 @@ ATTACK_REV_GRAD = 1
 ATTACK_CONSTANT = 2
 ATTACK_RANDOM = 3
 ATTACK_OMNISCIENT = 4
+ATTACK_ALIE = 5
+ATTACK_IPM = 6
+COLLUSION_ATTACKS = (ATTACK_ALIE, ATTACK_IPM)     # applied by the parameter server, not by the worker's push
 
 _ATTACK_CODES = {
     "none": ATTACK_NONE,
@@ -38,6 +50,8 @@ _ATTACK_CODES = {
     "constant": ATTACK_CONSTANT,
     "random": ATTACK_RANDOM,
     "omniscient": ATTACK_OMNISCIENT,
+    "alie": ATTACK_ALIE,
+    "ipm": ATTACK_IPM,
 }
 
 
@@ -106,3 +120,42 @@ def err_simulation(grad: np.ndarray, mode: str, cyclic: bool = False, *, magnitu
     if cyclic:
         return g + adv
     return adv if np.iscomplexobj(g) else adv.astype(g.dtype, copy=False)
+
+
+def alie_z_max(num_workers: int, worker_fail: int) -> float:
+    """ALIE's default z (Baruch et al., NeurIPS 2019, section 3): with ``s = floor(P/2 + 1) - f`` honest workers the
+    liars must win over, the largest z for which ``s`` of them are still expected to sit farther from the mean than the
+    lie, ``z = Phi^{-1}((P - s) / P)``.  Undefined (ValueError) when ``s <= 0``: the liars alone are a majority."""
+    P, f = int(num_workers), int(worker_fail)
+    s = (P // 2 + 1) - f
+    if P < 1 or s <= 0:
+        raise ValueError(f"ALIE's default z is undefined for {P} workers with {f} liars (s = floor(P/2 + 1) - f = {s} <= 0); "
+                         f"pass --alie-z")
+    return NormalDist().inv_cdf((P - s) / P)
+
+
+def collude(slots: np.ndarray, liars: Sequence[int], mode: str, param: float) -> np.ndarray:
+    """Oracle of the colluding attacks.  ``slots``: [P, D] worker gradients; ``liars``: 0-based rows that lie.  Returns an
+    fp64 copy of the slab whose liar rows all hold the same vector, computed in fp64 from the honest rows H (every other
+    row, ascending): ``mu - param * sigma`` for ``alie`` (``param`` = z), ``-param * mu`` for ``ipm`` (``param`` = epsilon),
+    with ``mu`` the mean and ``sigma`` the unbiased (ddof = 1) standard deviation of each coordinate over H.  Honest rows are
+    returned unchanged; non-finite honest values propagate per IEEE."""
+    out = np.array(slots, dtype=np.float64, copy=True)
+    P = out.shape[0]
+    lie = sorted({int(r) for r in liars})
+    if any(r < 0 or r >= P for r in lie):
+        raise ValueError(f"liar rows {lie} outside 0..{P - 1}")
+    honest = [r for r in range(P) if r not in lie]
+    if not lie or not honest:
+        return out
+    X = out[honest]
+    mu = X.sum(axis=0) / len(honest)
+    if mode == "alie":
+        sigma = np.sqrt(((X - mu) ** 2).sum(axis=0) / (len(honest) - 1)) if len(honest) > 1 else np.full_like(mu, np.nan)
+        v = mu - float(param) * sigma
+    elif mode == "ipm":
+        v = -float(param) * mu
+    else:
+        raise ValueError(f"unknown colluding attack {mode!r}")
+    out[lie] = v
+    return out

@@ -7,13 +7,15 @@ logging, ``--no-cuda`` forces the CPU/Gloo path) -- see DESIGN.md "flag semantic
 from __future__ import annotations
 
 import argparse
+import math
 from dataclasses import asdict, dataclass
 from typing import Optional
 
 APPROACHES = ("baseline", "maj_vote", "cyclic")
 MODES = ("normal", "geometric_median", "krum", "maj_vote", "coord_median", "trimmed_mean", "multi_krum")
 ROBUST_NVL_MAXP = 16            # P limit of coord_median / trimmed_mean / multi_krum on nvl (register budget of their kernels)
-ERR_MODES = ("rev_grad", "constant", "random", "omniscient", "none")
+ERR_MODES = ("rev_grad", "constant", "random", "omniscient", "alie", "ipm", "none")
+COLLUDING_ERR_MODES = ("alie", "ipm")   # every liar sends one vector built from the honest gradients, applied at the PS
 TRANSPORTS = ("nvl", "nccl", "nccl_flat", "gloo")
 
 
@@ -77,6 +79,8 @@ class JobConfig:
     push_ctas: int = 16             # CTAs of an overlapped bucket push (NVLink-bound: a handful of SMs saturates the link)
     worker_streams: int = 4         # >1: logical workers sharing a GPU run on (up to) this many concurrent CUDA streams
     zero_copy_grads: bool = True    # push reads gradients where autograd left them (pointer table), no flat gather
+    alie_z: Optional[float] = None  # --err-mode alie: the lie is mu - z * sigma; None = Baruch et al.'s z_max(P, worker_fail)
+    ipm_epsilon: float = 0.1        # --err-mode ipm: the lie is -epsilon * mu
 
     # ---- derived --------------------------------------------------------------------------
     def resolve(self, world_size: int) -> "JobConfig":
@@ -114,6 +118,8 @@ class JobConfig:
             if self.transport == "nvl" and P > ROBUST_NVL_MAXP:
                 raise ValueError(f"--mode {self.mode} on --transport nvl handles at most {ROBUST_NVL_MAXP} workers (got {P}); "
                                  f"use --transport nccl for more")
+        if self.err_mode in COLLUDING_ERR_MODES:
+            self._check_collusion()
         if self.compress and self.transport == "nvl" and self.err_mode == "omniscient":
             raise ValueError("--err-mode omniscient reads the honest slots in PS memory while they arrive; with --compress-grad "
                              "compress they only exist after the PS unpacked them -- pass --compress-grad None")
@@ -123,6 +129,34 @@ class JobConfig:
             self.dtype = "fp32"
             self.cuda_graphs = False
         return self
+
+    def _check_collusion(self) -> None:
+        P, f = self.num_workers, self.worker_fail
+        if self.approach == "cyclic":
+            raise ValueError(f"--err-mode {self.err_mode} is defined over real gradients; the cyclic code's adversary adds an "
+                             f"error to a complex codeword -- use another --approach")
+        for name, v in (("--alie-z", self.alie_z), ("--ipm-epsilon", self.ipm_epsilon)):
+            if v is not None and not math.isfinite(float(v)):
+                raise ValueError(f"{name} must be finite (got {v})")
+        if self.err_mode == "alie" and P - f < 2:
+            raise ValueError(f"--err-mode alie needs at least 2 honest workers for the standard deviation (got {P} workers, "
+                             f"worker_fail {f})")
+        if self.err_mode == "ipm" and P - f < 1:
+            raise ValueError(f"--err-mode ipm needs at least 1 honest worker (got {P} workers, worker_fail {f})")
+        if self.err_mode == "alie" and self.alie_z is None:
+            from .codes.adversary import alie_z_max
+            alie_z_max(P, f)                    # raises when the default z is undefined (the liars alone are a majority)
+
+    @property
+    def attack_param(self) -> float:
+        """z of ``--err-mode alie`` (``--alie-z``, else Baruch et al.'s default for P workers and worker_fail liars) or
+        epsilon of ``--err-mode ipm``."""
+        if self.err_mode == "ipm":
+            return float(self.ipm_epsilon)
+        if self.alie_z is not None:
+            return float(self.alie_z)
+        from .codes.adversary import alie_z_max
+        return alie_z_max(self.num_workers, self.worker_fail)
 
     @property
     def compress(self) -> bool:
@@ -170,7 +204,12 @@ def add_fit_args(parser: argparse.ArgumentParser) -> argparse.ArgumentParser:
       help="normal | geometric_median | krum | coord_median | trimmed_mean | multi_krum (baseline); normal | maj_vote (maj_vote)")
     a("--dataset", type=str, default=d.dataset)
     a("--comm-type", type=str, default=d.comm_type)
-    a("--err-mode", type=str, default=d.err_mode, help="rev_grad | constant | random | omniscient | none")
+    a("--err-mode", type=str, default=d.err_mode,
+      help="rev_grad | constant | random | omniscient | alie | ipm | none.  alie (Baruch et al., 2019) and ipm (Xie et al., "
+           "2019) collude: every liar sends mu - z * sigma / -epsilon * mu of the honest gradients (not with --approach cyclic)")
+    a("--alie-z", type=float, default=d.alie_z,
+      help="z of --err-mode alie (default: Phi^-1((P - s) / P) with s = floor(P/2 + 1) - worker_fail)")
+    a("--ipm-epsilon", type=float, default=d.ipm_epsilon, help="epsilon of --err-mode ipm")
     a("--approach", type=str, default=d.approach, help="baseline | maj_vote | cyclic")
     a("--num-aggregate", type=int, default=d.num_aggregate)
     a("--eval-freq", type=int, default=d.eval_freq)

@@ -109,6 +109,21 @@ def omniscient(grad_in: Addr, slot_stride: int, honest_mask: int, worker: int, m
     N.check(N.cuda().drc_omniscient(C.byref(a), grid, _stream()), "omniscient")
 
 
+def collude(layout: ArenaLayout, grad_in: Addr, slot_stride: int, P: int, adv_bitmap: Addr, adv_len: int, step_ptr: Addr,
+            mode: int, param: float, tile_range: Optional[tuple] = None) -> None:
+    """Colluding attack at the PS (csrc/cuda/collude.cu): the slots set in ``adv_bitmap[*step_ptr % adv_len]`` are all
+    overwritten with ``mu - param * sigma`` (``mode`` = ATTACK_ALIE) or ``-param * mu`` (ATTACK_IPM) of the other slots.
+    ``tile_range=(t0, t1)`` processes one bucket; an empty one launches nothing (tile_end 0 means "to the end" in the kernel)."""
+    dev = torch.device("cuda", torch.cuda.current_device())
+    t0, t1 = tile_range if tile_range is not None else (0, 0)
+    if tile_range is not None and t1 <= t0:
+        return
+    a = N.CollusionArgs(addr(grad_in), slot_stride, P, layout.tile_view(dev), int(t0), int(t1), addr(adv_bitmap), adv_len,
+                        addr(step_ptr), mode, param)
+    ntiles = (t1 - t0) if tile_range is not None else layout.ntiles
+    N.check(N.cuda().drc_collude(C.byref(a), max(1, min(ntiles, sm_count() * 8)), _stream()), "collude")
+
+
 # ------------------------------------------------------------------------------------------------ vote (K3)
 def vote(layout: ArenaLayout, grad_in: Addr, slot_stride: int, group_table: torch.Tensor, neq_mask: torch.Tensor,
          winner_slot: torch.Tensor, winner_member: Optional[torch.Tensor] = None, tile_range: Optional[tuple] = None,

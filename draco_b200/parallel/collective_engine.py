@@ -20,7 +20,7 @@ import torch
 import torch.distributed as dist
 
 from ..codes.adversary import generate_schedule
-from ..config import JobConfig
+from ..config import COLLUDING_ERR_MODES, JobConfig
 from ..data import TensorDataset
 from ..utils.codec import compress, decompress
 from ..utils.metrics import PhaseTimer, limit_host_threads
@@ -64,6 +64,8 @@ class CollectiveEngine:
         if self.is_ps:
             self.slots = torch.zeros(self.P, self.layout.total, dtype=wire, device=self.device)
             self.ps = TorchPS(cfg, self.layout, self.device, self.params_f32, self.groups, self.code)
+            if self.use_adv and cfg.err_mode in COLLUDING_ERR_MODES:    # the colluded vector keeps the slots' padding zero
+                self._valid = torch.from_numpy(self.layout.valid_mask()).to(self.device)
         self.compress = cfg.compress and self.device.type == "cpu"
         self.compress_gpu = cfg.compress and self.device.type == "cuda"
         self.bytes_up = 0
@@ -138,6 +140,19 @@ class CollectiveEngine:
         mean = self.slots[[h - 1 for h in honest]].mean(0)
         for w in liars:
             self.slots[w - 1].copy_(mean * self.cfg.attack_magnitude)
+
+    def _collude(self, step: int) -> None:
+        """--err-mode alie / ipm: every liar slot <- mu - z * sigma / -epsilon * mu of the honest slots, per coordinate, in fp64
+        (codes/adversary.py::collude), rounded into the fp32 slots.  Padding stays zero."""
+        liars = [w - 1 for w in range(1, self.P + 1) if self.schedule.is_adversary(w, step)]
+        honest = [r for r in range(self.P) if r not in liars]
+        if not liars or not honest:
+            return
+        X = self.slots[honest].double()
+        mu = X.mean(0)
+        param = self.cfg.attack_param
+        lie = mu - param * X.std(0) if self.cfg.err_mode == "alie" else -param * mu
+        self.slots[liars] = torch.where(self._valid, lie, 0.0).to(self.slots.dtype)
 
     def _exchange_gradients(self, step: int) -> None:
         """Per-tensor point-to-point: every remote worker -> PS."""
@@ -240,6 +255,8 @@ class CollectiveEngine:
         if self.is_ps:
             if self.use_adv and self.cfg.err_mode == "omniscient":
                 self._omniscient(step)
+            elif self.use_adv and self.cfg.err_mode in COLLUDING_ERR_MODES:
+                self._collude(step)
             with self._phase("t_decode"):                 # reference: "Method Time Cost"
                 grads = self.ps.aggregate(self.slots)
             with self._phase("t_update"):                 # reference: "Update Time Cost"

@@ -31,7 +31,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from ..codes.adversary import attack_code, generate_schedule
+from ..codes.adversary import ATTACK_OMNISCIENT, COLLUSION_ATTACKS, attack_code, generate_schedule
 from ..config import JobConfig
 from ..data import BatchPlan, TensorDataset
 from ..ops import conv as _conv_ops
@@ -177,7 +177,8 @@ class FusedEngine:
             self.worker = WorkerCompute(cfg, device, self.local_workers, plan, dataset, self.layout, self.params_f32, model)
             self.worker.step_dev = self.step_dev       # dropout masks are keyed by the device step (graph replays advance it)
         if self.is_ps:
-            self.ps = FusedPS(cfg, self.layout, device, self.params_f32, self.grad_in, self.groups, self.code)
+            self.ps = FusedPS(cfg, self.layout, device, self.params_f32, self.grad_in, self.groups, self.code,
+                              adv_bitmap=self.adv_bitmap)
             self.dst_ptrs = [mapA[p].ptr for p in self.place.worker_procs() if p != 0]
             self.param_flag_ptrs = [mapA[p].ptr + D * 4 for p in self.place.active_procs()]
         self._dbg_buf = (torch.zeros(D * self.esize // 4, dtype=torch.float32, device=device)
@@ -190,6 +191,13 @@ class FusedEngine:
         words): what the PS must find in slot ``w`` if every peer store of the real push landed."""
         K.push_encode(self.layout, g32, g16, self._dbg_buf.data_ptr(), flag=None, **push_kw)
         self._dbg_sums[w] = self._dbg_buf.view(torch.int32).sum(dtype=torch.int64)
+
+    def _dbg_sum_slots(self, tile_range) -> None:
+        """PS-side checksums of (one bucket of) every slot, taken before a colluding attack rewrites the liar slots."""
+        words = self.grad_in.view(torch.int32).view(self.P, -1)
+        if tile_range is not None:
+            words = words[:, tile_range[0] * K.N.TILE: tile_range[1] * K.N.TILE]
+        self._dbg_ps_sums += words.sum(1, dtype=torch.int64)
 
     def _verify_checksums(self, step: int) -> None:
         sums = torch.zeros(self.P, dtype=torch.int64, device=self.device)
@@ -304,7 +312,7 @@ class FusedEngine:
             torch.cuda.current_stream().wait_stream(self._ps_stream)
         elif self.is_ps:
             n += self._enqueue_ps_part()
-        if self.is_ps and self.debug_checksum:      # every gradient flag of this step has been waited for on this stream
+        if self.is_ps and self.debug_checksum and not self.ps.collusion:    # every gradient flag of this step has been waited for
             self._dbg_ps_sums = self.grad_in.view(torch.int32).view(self.P, -1).sum(1, dtype=torch.int64)
         K.step_add(self.step_dev, 1); n += 1
         return n
@@ -319,6 +327,10 @@ class FusedEngine:
             ps_phase.__enter__()
             nvtx.range_push("draco/ps: gather + decode + update + broadcast")            # reference: Method / Update time
             base = self.flagsB.data_ptr()
+            before_collude = None
+            if self.debug_checksum and self.ps.collusion:
+                self._dbg_ps_sums = torch.zeros(self.P, dtype=torch.int64, device=self.device)
+                before_collude = self._dbg_sum_slots
             if self.pipeline_ps:
                 nb = len(self.worker.buckets)
 
@@ -329,7 +341,7 @@ class FusedEngine:
 
                 n += self.ps.enqueue_step(self.step_dev, mc_params=self.mc_params, dst=[] if self.mc_params else self.dst_ptrs,
                                           flags=self.param_flag_ptrs, buckets=self.worker.buckets, wait_bucket=wait_bucket,
-                                          before_update=self._stamp_decode_done)
+                                          before_update=self._stamp_decode_done, before_collude=before_collude)
             else:
                 flags = [base + i * MAX_BUCKETS * FLAG_STRIDE for i in range(self.P)]
                 K.wait_flags(flags, self.step_dev, 0, self.error, cfg.spin_timeout_s, self.stamps_ps); n += 1
@@ -339,7 +351,7 @@ class FusedEngine:
                         self.codec.unpack(self.stage[i], slots[i]); n += 1
                 n += self.ps.enqueue_step(self.step_dev, mc_params=self.mc_params,
                                           dst=[] if self.mc_params else self.dst_ptrs, flags=self.param_flag_ptrs,
-                                          before_update=self._stamp_decode_done)
+                                          before_update=self._stamp_decode_done, before_collude=before_collude)
         if self.default_phases:
             K.stamp(self.stamps_phase, self.step_dev, 2); n += 1
         nvtx.range_pop()
@@ -386,7 +398,9 @@ class FusedEngine:
                      and self.schedule.is_adversary(w, step_host))
         push_kw = dict(step_ptr=self.step_dev, worker=w - 1, done_counter=self.push_counters[w:w + 1], coef=coef,
                        adv_bitmap=self.adv_bitmap, adv_len=len(self.schedule.ranks),
-                       attack=self.attack if self.attack != 4 else 0, magnitude=cfg.attack_magnitude, seed=cfg.seed,
+                       # omniscient / colluding liars push their honest gradient: their lie is made from the honest slots
+                       attack=0 if self.attack == ATTACK_OMNISCIENT or self.attack in COLLUSION_ATTACKS else self.attack,
+                       magnitude=cfg.attack_magnitude, seed=cfg.seed,
                        src_table=wc.ptr_dev[w] if wc.zero_copy else None)
         if self.overlap_push and not lying_now:
             # bucketed push on a side stream, overlapped with the rest of the backward pass

@@ -17,6 +17,7 @@ import numpy as np
 import torch
 
 from .. import _native as N
+from ..codes.adversary import COLLUSION_ATTACKS, attack_code
 from ..codes.cyclic import CyclicCode, search_w
 from ..codes.repetition import GroupPlan
 from ..config import JobConfig
@@ -57,11 +58,18 @@ class FusedPS:
     """Kernel-driven PS state for one job (lives on the PS GPU)."""
 
     def __init__(self, cfg: JobConfig, layout: ArenaLayout, device: torch.device, params: torch.Tensor,
-                 grad_in: torch.Tensor, groups: Optional[GroupPlan], code: Optional[CyclicCode]):
+                 grad_in: torch.Tensor, groups: Optional[GroupPlan], code: Optional[CyclicCode], *,
+                 adv_bitmap: Optional[torch.Tensor] = None):
         from ..ops import kernels as K
         self.K = K
         self.cfg, self.layout, self.device = cfg, layout, device
         self.P = cfg.num_workers
+        # --err-mode alie / ipm: the liar slots of the step (device bitmap per step, see codes/adversary.py) are overwritten
+        # by the collusion kernel after their gradients arrived and before the rule reads them
+        self.adv_bitmap = adv_bitmap
+        attack = attack_code(cfg.err_mode)
+        self.collusion = attack if adv_bitmap is not None and attack in COLLUSION_ATTACKS else 0
+        self.collusion_param = cfg.attack_param if self.collusion else 0.0
         self.params = params                       # fp32 [D] master copy (inside the exported region)
         self.grad_in = grad_in                     # fp32 [P, D] or complex64-as-fp32 [P, 2D]
         self.momentum = layout.new_arena(device)             # SGD momentum buffer / Adam first moment
@@ -109,13 +117,27 @@ class FusedPS:
         """Optimizer arenas beyond ``momentum`` (Adam second moment, AMSGrad maximum) for checkpoints."""
         return {"exp_avg_sq": self.exp_avg_sq, "max_exp_avg_sq": self.max_exp_avg_sq}
 
+    def collude(self, step_ptr: torch.Tensor, tile_range: Optional[tuple] = None, before=None) -> int:
+        """Colluding attack of the step on the slab (or one bucket of it): ``before(tile_range)`` runs first, while every
+        slot still holds what its worker pushed.  Returns the number of kernels launched (0 without such an attack)."""
+        if not self.collusion:
+            return 0
+        if before is not None:
+            before(tile_range)
+        self.K.collude(self.layout, self.grad_in, self.slot_stride, self.P, self.adv_bitmap, self.adv_bitmap.numel(),
+                       step_ptr, self.collusion, self.collusion_param, tile_range=tile_range)
+        return 1
+
     def enqueue_step(self, step_ptr: torch.Tensor, *, mc_params: Optional[int], dst: Sequence[int], flags: Sequence[int],
-                     grad_out: Optional[torch.Tensor] = None, buckets=None, wait_bucket=None, before_update=None) -> int:
+                     grad_out: Optional[torch.Tensor] = None, buckets=None, wait_bucket=None, before_update=None,
+                     before_collude=None) -> int:
         """Decode + update + broadcast for the step in ``*step_ptr``.  Returns the number of kernels launched.
 
         With ``buckets`` (the workers' push buckets, in arrival order) and ``wait_bucket(b)`` the PS is pipelined: bucket
         ``b`` is voted on, applied and broadcast as soon as every worker has pushed it, while the workers are still
-        back-propagating / pushing the later buckets; only the last bucket is on the critical path."""
+        back-propagating / pushing the later buckets; only the last bucket is on the critical path.  Under a colluding
+        attack each bucket (or the whole slab) first goes through the collusion kernel; ``before_collude(tile_range)`` is
+        called right before it."""
         K, L = self.K, self.layout
         before_update = before_update or (lambda: 0)      # called right before the (last) fused update + broadcast kernel
         common = dict(params=self.params, momentum=self.momentum, exp_avg_sq=self.exp_avg_sq, max_exp_avg_sq=self.max_exp_avg_sq,
@@ -125,6 +147,7 @@ class FusedPS:
         if buckets is not None and self.rule in ("mean", "vote") + COORDINATE_RULES:
             for bi, (t0, t1, idxs) in enumerate(buckets):
                 n += wait_bucket(bi)
+                n += self.collude(step_ptr, (t0, t1), before_collude)
                 fl = flags if bi == len(buckets) - 1 else []
                 if self.rule == "vote":
                     K.vote(L, self.grad_in, self.slot_stride, self.group_table, self.neq_mask, self.winner_slot,
@@ -146,6 +169,7 @@ class FusedPS:
                                        tile_range=(t0, t1), flags=fl, **common); n += 1
             return n
         common["flags"] = flags
+        n += self.collude(step_ptr, None, before_collude)
         _agg = K.aggregate_update
 
         def _update(*a, **kw):                             # every rule below ends in exactly one fused update kernel
